@@ -1,8 +1,11 @@
 """CPU-side checks of the boundary: the C-ABI library loads and exports every symbol the
 header declares; host-side module logic (constructors, state_dict schema, loud failure)."""
 import ctypes
+import importlib
+import json
 import os
 import re
+import sys
 
 import numpy as np
 import pytest
@@ -92,29 +95,79 @@ def test_product_package_never_imports_oracle():
             assert "oracle" not in src.replace("# oracle", ""), f"{fn} references the oracle"
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/models"), reason="reference checkout only exists in the build container")
-def test_patch_reference_rebinds_names():
-    done = S.patch_reference("/root/reference")
-    assert "models.SmaAt_UNet" in done
+# One module of the stand-in `models` package.  It binds the same nn.Module class names as the reference module of that
+# name; its model classes make the reference constructors' block calls, looking each name up when the constructor runs.
+_STANDIN_MODULE = '''\
+from torch import nn
+
+_LAYOUT = {layout!r}
+
+
+class _NotRebound(nn.Module):
+    def __init__(self, *args, **kwargs):
+        raise AssertionError(type(self).__name__ + " was built but patch_reference() did not rebind it")
+
+
+for _n in _LAYOUT["binds"]:
+    globals()[_n] = type(_n, (_NotRebound,), {{}})
+
+
+def _model_class(name, calls):
+    def __init__(self):
+        nn.Module.__init__(self)
+        for attr, block, args, kwargs in calls:
+            setattr(self, attr, globals()[block](*args, **kwargs))
+    return type(name, (nn.Module,), {{"__init__": __init__}})
+
+
+for _n, _m in _LAYOUT["models"].items():
+    globals()[_n] = _model_class(_n, _m["calls"])
+'''
+
+
+def _drop_models_package():
+    for name in [m for m in sys.modules if m == "models" or m.startswith("models.")]:
+        del sys.modules[name]
+
+
+@pytest.fixture
+def reference_layout(tmp_path, monkeypatch):
+    """A stand-in for the reference checkout's `models` package, written from tests/golden/patch_layout.json (recorded from
+    the unmodified reference by oracle/make_golden_patch.py).  Yields (root to pass to patch_reference, the layout)."""
+    with open(os.path.join(ROOT, "tests", "golden", "patch_layout.json")) as f:
+        layout = json.load(f)
+    pkg = tmp_path / "models"
+    pkg.mkdir()
+    (pkg / "__init__.py").write_text("")
+    for modname, entry in layout["modules"].items():
+        (pkg / (modname.split(".", 1)[1] + ".py")).write_text(_STANDIN_MODULE.format(layout=entry))
+    monkeypatch.setattr(sys, "path", list(sys.path))
+    _drop_models_package()
+    importlib.invalidate_caches()
+    yield str(tmp_path), layout
+    _drop_models_package()
+
+
+def test_patch_reference_rebinds_names(reference_layout):
+    root, layout = reference_layout
+    done = S.patch_reference(root)
+    assert {k: sorted(v) for k, v in done.items()} == layout["patched"]
     import models.SmaAt_UNet as msu
-    m = msu.SmaAt_UNet(12, 1)
+    m = msu.SmaAt_UNet()                                  # the reference's SmaAt_UNet(12, 1)
     assert type(m.inc) is S.DoubleConvDS and type(m.cbam3) is S.CBAM and type(m.up2) is S.UpDS and type(m.outc) is S.OutConv
     assert len(m.state_dict()) == 214
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/models"), reason="reference checkout only exists in the build container")
-def test_patch_reference_reaches_the_lightning_wrappers():
+def test_patch_reference_reaches_the_lightning_wrappers(reference_layout):
     """The Lightning wrapper classes (models/unet_precip_regression_lightning.py:86-208) import the block classes by name;
-    after patch_reference() their UNCHANGED constructors build B200 blocks and keep the reference's state_dict schema.
-    `lightning` / `torchmetrics` / `h5py` are not installed here: oracle/ref_stubs.py stands in for those imports only."""
-    from oracle import ref_stubs
+    after patch_reference() their UNCHANGED constructors build B200 blocks and keep the reference's state_dict schema."""
     from oracle.cases import smaat_unet_schema
-    ref_stubs.install()
-    done = S.patch_reference("/root/reference", strict=True)
+    root, layout = reference_layout
+    done = S.patch_reference(root, strict=True)
     assert "models.unet_precip_regression_lightning" in done
     import models.unet_precip_regression_lightning as L
     for cls, n_cbams in (("UNetDSAttention", 5), ("UNetDSAttention4CBAMs", 4), ("UNetDS", 0)):
-        m = getattr(L, cls)(hparams=ref_stubs.hparams(12, 1, 2))
+        m = getattr(L, cls)()                             # built with hparams(n_channels=12, n_classes=1, kernels_per_layer=2)
         assert type(m.inc) is S.DoubleConvDS and type(m.down4) is S.DownDS and type(m.up1) is S.UpDS and type(m.outc) is S.OutConv
         if n_cbams:
             assert type(m.cbam1) is S.CBAM

@@ -1,8 +1,12 @@
-"""bench.py contract (CPU part): the reference arm prints ONE JSON line with the keys the driver reads."""
+"""bench.py contract: the reference arm prints ONE JSON line with the keys a caller reads; the b200 arm times the
+requested steps, dumps what the last one computed (-m gpu) and fails loudly without a GPU."""
 import json
 import os
 import subprocess
 import sys
+
+import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -21,6 +25,20 @@ def test_reference_arm_prints_the_contract_line():
     assert d["e2e"] == {"value": d["value"], "unit": d["unit"], "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
     with open(os.path.join(ROOT, "BASELINE.json")) as f:
         assert d["metric"] == json.load(f)["metric"]
+
+
+@pytest.mark.gpu
+def test_b200_arm_times_the_requested_steps_and_dumps_the_last_output(tmp_path):
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "2", "--warmup", "3", "--no-train", "--no-alt",
+                          "--no-cpu-baseline", "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=900, cwd=ROOT)
+    assert out.returncode == 0, out.stderr[-2000:]
+    lines = [l for l in out.stdout.strip().splitlines() if l.startswith("{")]
+    assert len(lines) == 1
+    assert json.loads(lines[0])["steps"] == 2
+    assert sorted(os.listdir(tmp_path)) == ["output.npy"]
+    y = np.load(tmp_path / "output.npy")
+    assert y.shape == (32, 1, 288, 288) and y.dtype == np.float32
+    assert np.isfinite(y).all() and np.abs(y).max() > 0
 
 
 def test_b200_arm_fails_loudly_without_a_gpu():
